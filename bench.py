@@ -2,6 +2,7 @@
 """bench.py -- env-steps/s of the fused WheeledLab step (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload drift|elev|hound4wd] [--envs E] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one env.step() of the workload over E envs per GPU with synthetic U[-1,1]^2 actions from the counter-based
@@ -63,6 +64,8 @@ WORKLOADS = {
                  "kernel": "wl_step_duo_kernel (4WD action map)", "traffic_profile": "profiles/r02_ncu_step_hound_8192.txt"},
 }
 L2_BYTES = 126 * 1024 * 1024
+SET_BYTES_PER_ENV = 256                                        # state + parameters per env: 16 groups x 16 B (wl_state_bytes)
+DUMP_BYTES = 64 * 10**6                                        # --dump-outputs: all files together, .npy headers included
 
 
 def _peaks():
@@ -87,6 +90,27 @@ def _traffic(path):
                 val, unit = line.split("=")[1].split()[:2]
                 tot += float(val) * {"byte": 1, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9}.get(unit, 1)
     return tot or None
+
+
+def dump_outputs(outdir, outputs):
+    """--dump-outputs: what the last timed step returned ({name: torch or numpy array, one row per env}) as float32
+    <outdir>/<name>.npy.  When the rows exceed DUMP_BYTES together, every array keeps the same fixed, seeded sample of
+    envs (in env order)."""
+    import numpy as np
+    n = len(next(iter(outputs.values())))
+    row_bytes = sum(4 * math.prod(a.shape[1:]) for a in outputs.values())
+    keep = (DUMP_BYTES - 256 * len(outputs)) // row_bytes     # (256 B: more than an .npy header takes)
+    rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False)) if n > keep else None
+    Path(outdir).mkdir(parents=True, exist_ok=True)
+    for name, a in outputs.items():
+        if hasattr(a, "cpu"):                                  # a torch tensor: only the kept rows leave the device
+            if rows is not None:
+                import torch
+                a = a[torch.from_numpy(rows).to(a.device)]
+            a = a.cpu().numpy()
+        elif rows is not None:
+            a = a[rows]
+        np.save(Path(outdir) / f"{name}.npy", np.ascontiguousarray(a, dtype=np.float32))
 
 
 class ClockSampler:
@@ -244,25 +268,24 @@ def run_reference(args):
     envs = (args.envs or w["envs"]) * max(1, args.gpus)
     threads, probe = _pick_threads(args.workload, envs, args.seed)
     orc = _cpu_oracle(args.workload, envs, args.seed, threads)
-    # one reference "step" = `reps` consecutive env.steps (a bounded sample sized so that K steps take >= ~1 s in total)
-    probe_steps, probe_el = _time_oracle(orc, args.warmup, 5, 0.2, 2.0)
-    per = probe_el / probe_steps
-    reps = max(1, math.ceil(1.0 / (per * args.steps)))
     acts = [orc.synth_actions(t) for t in range(8)]
-    t = args.warmup + probe_steps
+    for t in range(args.warmup):
+        orc.step(acts[t % 8], t)
     t0 = time.perf_counter()
-    for k in range(args.steps * reps):
-        orc.step(acts[k % 8], t + k)
+    for k in range(args.steps):
+        out = orc.step(acts[k % 8], args.warmup + k)
     el = time.perf_counter() - t0
-    val = envs * args.steps * reps / el
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("obs", "rewards", "terminated", "truncated"), out)))
+    val = envs * args.steps / el
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": 1e3 * el / (args.steps * reps), "higher_is_better": True, "scaling": "weak",
+        "warmup": args.warmup, "ms_per_step": 1e3 * el / args.steps, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"{w['label']}: {envs} envs (CPU, one box)", "envs_per_step": envs, "same_config": True,
                    "note": "PhysX is not runnable here; this is the CPU restatement of the same step (oracle/wl_oracle.c)"},
         "cpu_baseline": {"value": val, "unit": UNIT, "cores": threads, "kind": "port", "thread_probe": probe,
-                         "sample": f"{envs} envs x {args.steps} steps x {reps} env-steps each, OpenMP {threads} threads (best of 1/4, 1/2, 1 x "
+                         "sample": f"{envs} envs x {args.steps} steps, OpenMP {threads} threads (best of 1/4, 1/2, 1 x "
                                    f"{_physical_cores()} physical cores; {os.cpu_count()} logical), OMP_PROC_BIND=close, {el:.2f} s timed"},
         "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
@@ -321,9 +344,11 @@ def run_ours(args):
         return float(tt.item())
 
     # ---- M independent env sets: the working set (state + parameters) exceeds L2, so round-robin stepping is cold ----
+    # M follows the nominal SET_BYTES_PER_ENV, not this build's buffer size: which env set runs step k, with which seed
+    # and history, then depends on the arguments only, and --dump-outputs of two builds can be compared
     sim0 = wl.WheeledSim(mk(), dev)
     set_bytes = sim0._buf.numel() * 4
-    M = max(4, math.ceil(2.2 * L2_BYTES / set_bytes))
+    M = max(4, math.ceil(2.2 * L2_BYTES / (SET_BYTES_PER_ENV * E)))
     sims = [sim0] + [wl.WheeledSim(mk(1000 * m), dev) for m in range(1, M)]
     for s in sims:
         s.startup(); s.reset(None, 0)
@@ -474,6 +499,10 @@ def run_ours(args):
     e1.record()
     barrier()
     tot_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:                      # before anything else writes into the slabs
+        last = W + K - 1
+        obs, rew, term, trunc = slabs[(last // T_ROLL) % n_slabs].step_outputs(last % T_ROLL)
+        dump_outputs(args.dump_outputs, {"obs": obs, "rewards": rew, "terminated": term, "truncated": trunc})
     launches = (sum(s.launch_count for s in sims) - l0) if graph is None else K
     n_exchanges = len(gev)
     # duration of one exchange on its own (eager, outside the timed region): all-gather ms / barrier ms
@@ -733,6 +762,10 @@ def main():
                     help="N > 1 slab exchange: fused into the step kernel as NVSwitch-multicast stores (mcast; auto for the Drift family, "
                          "falling back to per-peer stores = fanout, then to NCCL), copy-engine pull over symmetric memory (ce; auto "
                          "for Elevation), or NCCL all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (observations, "
+                    "rewards, terminated, truncated) as float32 DIR/<name>.npy (<= 64 MB: a seeded sample of envs when larger).  "
+                    "Compares builds run with the same arguments and --impl; the two --impl arms step different env sets, "
+                    "so their dumps are not comparable with each other")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3

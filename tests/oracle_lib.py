@@ -3,6 +3,7 @@ from __future__ import annotations
 
 import ctypes as C
 import subprocess
+import tempfile
 from pathlib import Path
 
 import numpy as np
@@ -11,13 +12,20 @@ ROOT = Path(__file__).resolve().parent.parent
 ODIR = ROOT / "oracle"
 
 
-def _ensure_built(native=False):
-    targets = ["libwl_oracle.so", "libwl_oracle_f64.so"] + (["libwl_oracle_native.so"] if native else [])
-    subprocess.run(["make", "-C", str(ODIR), *targets], check=True, stdout=subprocess.DEVNULL)
+def _ensure_built():
+    subprocess.run(["make", "-C", str(ODIR), "libwl_oracle.so", "libwl_oracle_f64.so"], check=True, stdout=subprocess.DEVNULL)
 
 
-def _load(name):
-    lib = C.CDLL(str(ODIR / name))
+def _load_native():
+    """The -march=native build is compiled for the host that loads it, in a temporary directory (the tree may be
+    read-only); the file is removed once it is mapped, so every process that loads it pays the few-second compile."""
+    with tempfile.TemporaryDirectory(prefix="wl_oracle_native_") as d:
+        subprocess.run(["make", "-C", str(ODIR), f"NATIVE_DIR={d}", f"{d}/libwl_oracle_native.so"], check=True, stdout=subprocess.DEVNULL)
+        return _load(Path(d) / "libwl_oracle_native.so")
+
+
+def _load(path):
+    lib = C.CDLL(str(path))
     vp, i32, i64, u32, u64 = C.c_void_p, C.c_int32, C.c_int64, C.c_uint32, C.c_uint64
     lib.wlo_create.restype = vp
     lib.wlo_create.argtypes = [vp, vp]
@@ -54,8 +62,11 @@ _libs = {}
 
 def get_lib(kind="f32"):
     if kind not in _libs:
-        _ensure_built(native=(kind == "native"))
-        _libs[kind] = _load({"f32": "libwl_oracle.so", "f64": "libwl_oracle_f64.so", "native": "libwl_oracle_native.so"}[kind])
+        if kind == "native":
+            _libs[kind] = _load_native()
+        else:
+            _ensure_built()
+            _libs[kind] = _load(ODIR / {"f32": "libwl_oracle.so", "f64": "libwl_oracle_f64.so"}[kind])
     return _libs[kind]
 
 
